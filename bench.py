@@ -105,7 +105,7 @@ def _pool_init(adj_blob, cv, mnph, use_ref):
     _G["cv"], _G["mnph"], _G["ref"] = cv, mnph, None
     if use_ref:
         from oracle import ref_shim
-        m = ref_shim.load()                      # the reference's own util_functions.py (oracle/_ref or /root/reference)
+        m = ref_shim.load()                      # the reference's own util_functions.py (oracle/_ref)
         _G["ref"] = m
         _G["idx"] = (m.SparseRowIndexer(A), m.SparseColIndexer(A.tocsc()))
     else:
@@ -259,7 +259,7 @@ def run_reference(args, ds, B, rank):
 
 def cpu_baseline_dict(r):
     # kind: the model half is a restatement (PyG 1.4.2 is not installable here), so the arm as a whole is a port;
-    # the extraction half runs the reference's own code whenever oracle/_ref (or /root/reference) is present
+    # the extraction half runs the reference's own code whenever oracle/_ref is present
     return {"value": r["value"], "unit": "subgraphs/s", "cores": r["cores"], "kind": "port",
             "extraction_kind": r["extraction_kind"], "model_kind": "port (PyG 1.4.2 RGCNConv restated)",
             "sample": r["sample"], "extraction_subgraphs_per_s": r["extraction_subgraphs_per_s"],
@@ -352,6 +352,26 @@ def batch_stats(ds, engine, idx_list):
         for k in range(len(idx)):
             tot["Du"] += int(rowdeg[nu[k, :cu[k]]].sum())
     return tot
+
+
+def step_outputs(eng, model, opt):
+    """Host copies of what a caller of the timed train step receives after its last step: the step's loss, the
+    updated parameters and the Adam moments, named by the model's state_dict keys."""
+    # last_loss is the tensor the step graphs were captured with; replays of either pipeline slot write into it because
+    # the model's workspace (and its loss) is keyed by batch shape, not by slot
+    out = {"loss": eng.last_loss.detach().float().cpu().numpy().reshape(-1)}
+    for name, p in model.named_parameters():
+        out["param." + name] = p.detach().float().cpu().numpy()
+        out["adam_exp_avg." + name] = opt.state[p]["exp_avg"].float().cpu().numpy()
+        out["adam_exp_avg_sq." + name] = opt.state[p]["exp_avg_sq"].float().cpu().numpy()
+    return out
+
+
+def write_outputs(path, outputs):
+    """``path``/<name>.npy per array (float32, a few hundred KB in all)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def run_ours(args):
@@ -458,6 +478,7 @@ def run_ours(args):
     clk = clocks.stop()
     per_step = np.array([a.elapsed_time(b) for a, b in zip(ev0, ev1)])
     dev_ms = float(per_step.sum())
+    outputs = step_outputs(eng, model, opt) if args.dump_outputs and rank == 0 else None
     if os.environ.get("IGMC_BENCH_DEBUG"):
         span = ev0[0].elapsed_time(ev1[-1])
         gaps = np.array([ev1[k].elapsed_time(ev0[k + 1]) for k in range(K - 1)])
@@ -509,9 +530,8 @@ def run_ours(args):
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         e2e_runs.append(float(t.item()))
-        if zc:
-            assert K <= eng.LOSS_RING
-            for k in range(K):
+        if zc:   # the ring keeps the losses of the last LOSS_RING updates
+            for k in range(max(0, K - eng.LOSS_RING), K):
                 loss_host[k] = eng.loss_of_update(u0 + k)
     e2e_s = min(e2e_runs)
     eng.check()
@@ -615,6 +635,8 @@ def run_ours(args):
             "batch_stats": {k: v / stats["B"] for k, v in stats.items() if k != "B"},
             "wall_s_timed_region": wall,
         }
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
     if world > 1:
         # NCCL communicators that were captured into CUDA graphs do not tear down reliably
         # (destroy_process_group was observed to hang): drop the graphs, align the ranks, and let main() leave
@@ -636,7 +658,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=12)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss, parameters and Adam moments of the last timed step "
+                         "as DIR/<name>.npy (float32); the inputs are seeded, so runs with the same arguments compare "
+                         "output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     # stdout carries exactly ONE line (the JSON): anything a library prints to fd 1 during the run (NCCL's version
     # banner, for one) is sent to stderr, and the result is written to the saved descriptor at the end

@@ -6,9 +6,8 @@ Python >= 3.11 ``random.sample`` refuses sets (reference line 223-229 passes
 sets), so calls are wrapped to pass ``tuple(population)`` which is what
 CPython <= 3.10 did internally.  Nothing else is changed.
 
-This module is used by ``tests/golden/make_golden.py`` and by the optional
-``test_oracle_vs_reference`` tests (skipped when /root/reference is absent, as
-on the GPU box).
+This module is used by the generators under ``tests/golden/`` (which store
+the reference's outputs for the tests) and by the CPU arm of ``bench.py``.
 """
 import importlib.util
 import os
@@ -16,13 +15,12 @@ import random
 import sys
 import types
 
-# the reference checkout (this container), else the vendored copy oracle/make_ref.py placed under oracle/_ref/
-# (git-ignored build product that travels to the GPU box with the snapshot)
+# the copy build() places under oracle/_ref/ (oracle/make_ref.py); without it, a reference checkout named by
+# IGMC_REFERENCE_DIR (for the golden-data generators run before a build)
 _VENDORED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
-REF_DIR = os.environ.get("IGMC_REFERENCE_DIR", "/root/reference")
-if not os.path.isfile(os.path.join(REF_DIR, "util_functions.py")) and \
-        os.path.isfile(os.path.join(_VENDORED, "util_functions.py")):
-    REF_DIR = _VENDORED
+REF_DIR = _VENDORED
+if not os.path.isfile(os.path.join(_VENDORED, "util_functions.py")) and os.environ.get("IGMC_REFERENCE_DIR"):
+    REF_DIR = os.environ["IGMC_REFERENCE_DIR"]
 
 
 def available():

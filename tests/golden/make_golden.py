@@ -1,6 +1,7 @@
 """Generate tests/golden/*.npz from the UNMODIFIED reference extraction code.
 
-Run in the build container only (needs /root/reference):
+Needs the reference's code: oracle/_ref/ as build() leaves it, or ``IGMC_REFERENCE_DIR`` naming a checkout
+(``oracle/ref_shim.py``):
 
     python tests/golden/make_golden.py
 
@@ -23,6 +24,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
 from oracle import ref_shim  # noqa: E402
 from igmc_b200.data import synth_ratings, build_adj  # noqa: E402
+from tests.helpers import reference_case_tag  # noqa: E402
 
 KEYS = ("u_nodes", "v_nodes", "u", "v", "r", "node_labels")
 
@@ -116,7 +118,39 @@ def main():
         rnd[tag + "__cv"] = cvv
     rnd["tags"] = np.array([s[0] for s in specs])
     np.savez_compressed(os.path.join(HERE, "random_cases.npz"), **rnd)
+    write_live_cases()
     print("wrote", os.listdir(HERE))
+
+
+def write_live_cases():
+    """reference_cases.npz: 40 pairs per (h, mnph) of tests/test_oracle_extract.py::test_live_reference, with the
+    reference's canonical subgraphs and the shapes / label of the PyG Data it built."""
+    out = {}
+    for h, mnph in LIVE_SPECS:
+        tag = reference_case_tag(h, mnph)
+        u, v, lab = synth_ratings(50, 45, 420, 5, seed=99 + h)
+        A = build_adj(u, v, lab, 50, 45)
+        cv = np.array([1, 2, 3, 4, 5.0])
+        idx = ref_shim.make_indexers(A)
+        random.seed(5)
+        cases, x_shape, n_edges, y = [], [], [], []
+        for c in range(40):
+            canon, raw = ref_shim.extract_ref_canonical(A, int(u[c]), int(v[c]), int(lab[c]), cv, h, 1.0, mnph, idx)
+            data = raw[-1]
+            cases.append(canon)
+            x_shape.append(tuple(data.x.shape))
+            n_edges.append(data.edge_index.shape[1])
+            y.append(float(data.y))      # the label as the reference's PyG Data carries it
+        for k, val in pack(cases).items():
+            out["%s__%s" % (tag, k)] = val
+        out[tag + "__coo"] = np.array([u, v, lab], np.int64)
+        out[tag + "__x_shape"] = np.array(x_shape, np.int64)
+        out[tag + "__n_edges"] = np.array(n_edges, np.int64)
+        out[tag + "__data_y"] = np.array(y, np.float64)
+    np.savez_compressed(os.path.join(HERE, "reference_cases.npz"), **out)
+
+
+LIVE_SPECS = ((1, None), (1, 6), (2, None), (2, 3))
 
 
 if __name__ == "__main__":

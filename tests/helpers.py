@@ -85,6 +85,11 @@ def batch_equal(b, ob):
     return out
 
 
+def reference_case_tag(h, mnph):
+    """key prefix of one (h, max_nodes_per_hop) group in tests/golden/reference_cases.npz"""
+    return "h%d_m%s" % (h, "none" if mnph is None else mnph)
+
+
 def load_flixster_cases():
     """(dataset dict, pairs [3,n], list of canonical dicts) of tests/golden/flixster_cases.npz: outputs of the
     reference's own subgraph_extraction_labeling on 64 pairs of the REAL flixster split (h=1, no sampling)."""

@@ -3,8 +3,8 @@
 ``eval(dataset_class)(...)``, ``IGMC(...)``, ``train_multiple_epochs`` with its ``logger`` (log.txt + checkpoints) and
 the checkpoint ensemble of ``test_once`` - with the data loaders stubbed by a synthetic split (tests/main_stubs).
 
-Main.py is taken from /root/reference when present, else from oracle/_ref/ (the git-ignored copy oracle/make_ref.py
-makes, which travels to the GPU box); without either the test is skipped."""
+Main.py is read from oracle/_ref/, the git-ignored copy that build() places through oracle/make_ref.py when it finds a
+checkout of the reference; without it the test is skipped (the reference's source is not part of this repository)."""
 import os
 import re
 import subprocess
@@ -18,11 +18,8 @@ pytestmark = pytest.mark.gpu
 
 
 def _main_py():
-    for d in ("/root/reference", os.path.join(ROOT, "oracle", "_ref")):
-        p = os.path.join(d, "Main.py")
-        if os.path.isfile(p):
-            return p
-    return None
+    p = os.path.join(ROOT, "oracle", "_ref", "Main.py")
+    return p if os.path.isfile(p) else None
 
 
 @pytest.mark.skipif(_main_py() is None, reason="reference Main.py not available (run oracle/make_ref.py)")
